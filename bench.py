@@ -2,7 +2,7 @@
 """bench.py -- rendered faces/sec of the FENeRF volumetric render hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model A|B]
-                    [--precision guard|fast|exact] [--no-graph] [--quick]
+                    [--precision guard|fast|exact] [--no-graph] [--quick] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic latents: BASELINE.json configs[1]
 -- 128x128 image, 24 (+24 hierarchical) samples per ray, batch 4 per GPU, forward-only -- through
@@ -12,6 +12,11 @@ N(0,1); camera poses gaussian (h_stddev 0.3, v_stddev 0.155); nerf_noise 0.  Eve
 end to end, per model and precision mode) starts from the same device state: queue drained, SETTLE_S
 of idle, W warm-up steps, then exactly K timed steps (StepRunner.settle says why).  One JSON line on
 stdout (rank 0).  Nothing here reads /root/reference.
+
+--dump-outputs DIR writes what the headline arm's last timed step returned to its caller: DIR/pixels.npy
+(every rank's frames, as read on the host) and DIR/poses.npy, float32.  The latents, the weights and the
+seed of the device RNG are fixed, so the same arguments give the same inputs on every run and two builds can
+be compared output for output.
 """
 import argparse
 import json
@@ -28,12 +33,14 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
     if p not in sys.path:
         sys.path.insert(0, p)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 FLOP_PER_POINT = {"A": 1053696, "B": 1341440}   # SURVEY.md section 8d (B: label chain pre-multiplied)
 MODEL_NAME = {"A": "ImplicitGenerator3d+TALLSIREN", "B": "DoubleImplicitGenerator3d+TextureEmbeddingPiGAN256SEMANTICDISENTANGLE_DIM_96"}
 IMG, STEPS_PER_RAY, BATCH_PER_GPU = 128, 24, 4
 SETTLE_S = 1.0      # idle time in front of every timed arm (StepRunner.settle)
+DUMP_BYTES = 63 << 20   # --dump-outputs stays under 64 MB in all
 
 
 def metadata(img_size=IMG):
@@ -241,6 +248,7 @@ class StepRunner:
         self.copy_stream = torch.cuda.Stream(device=device)
         self.host_sink = 0.0
         self.first_e2e = 0
+        self.last_out = None
         self.graph = None
         if use_graph:
             with torch.no_grad():
@@ -261,13 +269,13 @@ class StepRunner:
             # stage[i & 1] was last read by the D2H of step i-2: long finished, but keep the order explicit
             torch.cuda.current_stream().wait_event(self.out_done[i & 1])
         if self.graph is not None:
-            frames = self.graph(*self.lat_host[k])                 # H2D straight into the captured input buffers
-            frames = frames[0]
+            out = self.graph(*self.lat_host[k])                    # H2D straight into the captured input buffers
         else:
             zs = tuple(z.to(self.device, non_blocking=True) for z in self.lat_host[k])
             with torch.no_grad():
-                frames = self.gen(*zs, **self.md)[0]
-        allf = self.gatherer.gather(frames)
+                out = self.gen(*zs, **self.md)
+        self.last_out = out                                        # (frames, poses), as the generator returns them
+        allf = self.gatherer.gather(out[0])
         self.stage[i & 1].copy_(allf)
         self.frames_ready[i & 1].record()
         self.copy_stream.wait_event(self.frames_ready[i & 1])
@@ -340,12 +348,19 @@ class StepRunner:
         return sum(z.numel() * 4 for z in self.lat_host[0]), self.out_host[0].numel() * 4
 
 
-def measure_model(args, model, world, rank, local, steps, warmup, precision=None, sustained_s=0.0, roofline=True):
+def measure_model(args, model, world, rank, local, steps, warmup, precision=None, sustained_s=0.0, roofline=True,
+                  keep_outputs=False):
     device = torch.device("cuda", local)
     n_batches = min(steps + warmup, 64)
     r = StepRunner(args, model, world, rank, device, n_batches, precision=precision, use_graph=not args.no_graph)
     ms_step, _ = r.time_resident(steps, warmup)
     ms_e2e = r.time_e2e(steps, warmup)
+    outputs = None
+    if keep_outputs:
+        # the last timed step: its frames as the host read them, its poses from every rank
+        from fenerf_b200.dist import gather_frames
+        outputs = {"pixels": r.out_host[(warmup + steps - 1) & 1].float().numpy().copy(),
+                   "poses": gather_frames(r.last_out[1]).float().cpu().numpy()}
     B = BATCH_PER_GPU
     h2d, d2h = r.bytes_per_step()
     lps = r.launches_per_step()
@@ -367,7 +382,24 @@ def measure_model(args, model, world, rank, local, steps, warmup, precision=None
                             "ms_per_step": ms_long, "clocks": clocks}
     if roofline:
         out["roofline"] = field_roofline(r.gen, args, model, r.precision, r.lat_dev[0], metadata(), device)
+    if outputs is not None:
+        out["outputs"] = outputs
     return out
+
+
+def dump_outputs(out_dir, outputs):
+    """DIR/<name>.npy per array.  Past DUMP_BYTES a fixed, seeded subset of the images is kept (sorted; DIR/image_index.npy
+    holds their indices)."""
+    os.makedirs(out_dir, exist_ok=True)
+    pixels, poses = outputs["pixels"], outputs["poses"]
+    n = pixels.shape[0]
+    keep = max(1, min(n, DUMP_BYTES // (pixels[0].nbytes + poses[0].nbytes)))
+    if keep < n:
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        pixels, poses = pixels[idx], poses[idx]
+        np.save(os.path.join(out_dir, "image_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "pixels.npy"), pixels)
+    np.save(os.path.join(out_dir, "poses.npy"), poses)
 
 
 def measure_train_step(args, world, rank, local):
@@ -427,8 +459,10 @@ def run_ours(args, world, rank, local):
     ops.set_default_precision(args.precision)
     torch.manual_seed(4242 + rank)
     sampler = ClockSampler(local) if rank == 0 else None
-    main = measure_model(args, args.model, world, rank, local, args.steps, args.warmup, sustained_s=0.0)
+    main = measure_model(args, args.model, world, rank, local, args.steps, args.warmup, sustained_s=0.0,
+                         keep_outputs=args.dump_outputs is not None)
     clocks = sampler.stop() if sampler else None
+    outputs = main.pop("outputs", None)
     extras = {}
     if not args.quick:
         other = "B" if args.model == "A" else "A"
@@ -453,6 +487,8 @@ def run_ours(args, world, rank, local):
                 extras["train_step"] = {"error": repr(e)[:300]}
     if rank != 0:
         return
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     line = {
         "metric": "rendered faces/sec at 128px x 24 samples/ray", "value": main["value"], "unit": "faces/s",
         "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "ms_per_step": main["ms_per_step"],
@@ -560,7 +596,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="run the step eagerly instead of as a captured CUDA graph")
     ap.add_argument("--quick", action="store_true", help="headline numbers only (no sustained run / other model / modes / train step)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's frames and poses as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         world, rank = int(os.environ.get("WORLD_SIZE", "1")), int(os.environ.get("RANK", "0"))

@@ -1,8 +1,7 @@
 """Import shim for the UNMODIFIED reference at /root/reference (test infrastructure only).
 
-Used only by ``tests/golden/make_goldens.py`` and ``tests/test_oracle_vs_reference.py`` in the
-build container; ``/root/reference`` does not exist on the GPU box, so nothing on the product path
-and nothing under ``-m gpu`` imports this module.
+Used only by ``tests/golden/make_goldens.py`` and ``tools/port_vs_reference.py``: the tests compare
+with what ``make_goldens.py`` stored, so no test and nothing on the product path imports this module.
 
 The reference has four dead imports that are not installable here (SURVEY.md section 8c):
 ``matplotlib.pyplot`` (generators/volumetric_rendering.py:12), ``numpy.lib.type_check.imag``

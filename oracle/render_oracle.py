@@ -12,9 +12,8 @@ reference span it follows (paths relative to the reference root).
 How it is pinned: the reference holds no tests or golden vectors for this path (SURVEY.md
 section 4), so the pin is the unmodified reference itself, imported in the build container:
 ``tests/golden/make_goldens.py`` (committed) runs it on fixed seeds and stores its outputs under
-``tests/golden/``; ``tests/test_oracle.py`` checks this oracle against those files everywhere, and
-``tests/test_oracle_vs_reference.py`` checks bit-equality against the live reference where
-``/root/reference`` exists.
+``tests/golden/``; ``tests/test_oracle.py`` checks this oracle against those files within a
+cross-host tolerance, and ``tests/test_oracle_vs_reference.py`` checks bit-equality with them.
 
 RNG: every random draw goes through a ``Draws`` object so that a run can be recorded on the CPU
 and replayed, tensor for tensor, into the CUDA path (CPU and CUDA generators differ).

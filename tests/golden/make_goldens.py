@@ -52,6 +52,7 @@ def main():
     ref_generators, ref_siren, _ = ref_shim.load()
     out_dir = os.path.dirname(os.path.abspath(__file__))
     only = set(sys.argv[1:])                       # optional: case names to (re)generate
+    torch.set_num_threads(_cases.GOLDEN_THREADS)
     for case in _cases.CASES:
         if only and case.name not in only:
             continue
@@ -210,9 +211,41 @@ def part_forward_goldens():
                                                         os.path.getsize(path) / 1024))
 
 
+def pickle_goldens():
+    """tests/golden/ref_pickle_<A|D>.npz: whole-module checkpoints written by the reference's own classes
+    (train_double_latent_semantic.py:523 style) for tests/test_dropin.py.  What those tests check is the pickle's
+    structure (module paths, attribute names, parameter order) and that every state_dict entry lands on the right
+    tensor, so each state_dict tensor is first filled with its own constant (index + 1) / 64: the file then deflates
+    from ~10 MB to ~50 KB.  `checkpoint` holds the torch.save bytes, `meta` those of {names, state}."""
+    import io
+    ref_generators, ref_siren, _ = ref_shim.load()
+    out_dir = os.path.dirname(os.path.abspath(__file__))
+    for model in ("A", "D"):
+        torch.manual_seed(0)
+        if model == "A":
+            gen = ref_generators.ImplicitGenerator3d(ref_siren.TALLSIREN, 256, 4)
+        else:
+            gen = ref_generators.DoubleImplicitGenerator3d(ref_siren.SIRENBASELINESEMANTICDISENTANGLE, 256, 256, 22)
+        gen.set_device("cpu")
+        gen.step, gen.epoch = 1234, 7
+        with torch.no_grad():
+            for i, t in enumerate(gen.state_dict().values()):
+                t.fill_((i + 1) / 64)
+        ckpt, meta = io.BytesIO(), io.BytesIO()
+        torch.save(gen, ckpt)
+        torch.save({"names": [n for n, _ in gen.named_parameters()], "state": gen.state_dict()}, meta)
+        path = os.path.join(out_dir, "ref_pickle_%s.npz" % model)
+        np.savez_compressed(path, checkpoint=np.frombuffer(ckpt.getvalue(), np.uint8),
+                            meta=np.frombuffer(meta.getvalue(), np.uint8))
+        print("%-28s %d + %d bytes -> %s (%.1f KB)" % ("ref_pickle_" + model, len(ckpt.getvalue()), len(meta.getvalue()),
+                                                       os.path.basename(path), os.path.getsize(path) / 1024))
+
+
 if __name__ == "__main__":
     if sys.argv[1:2] == ["--part"]:
         part_forward_goldens()
+    elif sys.argv[1:2] == ["--pickles"]:
+        pickle_goldens()
     elif sys.argv[1:2] == ["--grads"]:
         grad_goldens()
         frequency_grad_goldens()
